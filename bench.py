@@ -60,6 +60,9 @@ def parse_args():
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--cpu-sample", type=int, default=256 << 20, help="bytes of the workload the in-line CPU baseline is timed on")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step returned (compressed blob, chunk directory, "
+                         "decoded symbols; seeded samples of the large ones) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -317,9 +320,30 @@ class Rig:
         return t.tolist()
 
 
-def measure(rig, workload, n, chunk, steps, warmup, e2e_steps, headline):
+DUMP_BYTES = 16_000_000        # per written array; at most four arrays, so a dump stays within 64 MB
+
+
+def dump_outputs(dump_dir, outputs):
+    """Write each device array as <dump_dir>/<name>.npy: float64 when its values could exceed float32's 24-bit exact
+    range (the directory's byte offsets), float32 otherwise.  An array with more elements than fit DUMP_BYTES is
+    reduced to the elements at distinct sorted positions drawn from a generator seeded with 0, so two runs with the
+    same arguments write the same positions."""
+    import torch
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.reshape(-1)
+        dtype = np.float64 if t.dtype == torch.int64 else np.float32
+        keep = DUMP_BYTES // np.dtype(dtype).itemsize
+        if t.numel() > keep:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), keep, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(dump_dir, name + ".npy"), t.cpu().numpy().astype(dtype))
+
+
+def measure(rig, workload, n, chunk, steps, warmup, e2e_steps, headline, dump_dir=None):
     """One workload on every rank: bit-exact check, K timed round trips (device-resident, CUDA events on the
-    context's stream, max over ranks), the host-buffer e2e number, and -- for the headline -- the blob gather."""
+    context's stream, max over ranks), the host-buffer e2e number, and -- for the headline -- the blob gather.
+    With `dump_dir`, rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     torch, rb, ctx, dev, world = rig.torch, rig.rb, rig.ctx, rig.dev, rig.world
     coder_name, sb, kind, stands_for = WORKLOADS[workload]
     coder = {"word": rb.CODER_WORD, "alias": rb.CODER_ALIAS, "rans64": rb.CODER_RANS64, "blocks": rb.CODER_WORD}[coder_name]
@@ -392,6 +416,11 @@ def measure(rig, workload, n, chunk, steps, warmup, e2e_steps, headline):
     ctx.sync()
     if not torch.equal(out, data):
         raise SystemExit(f"bench.py: {workload}: timed round trip is NOT bit-exact")
+    if dump_dir and rig.rank == 0:
+        outputs = {"blob": blob[:blob_size], "offsets": offsets, "decoded": out}
+        if blocks:
+            outputs["block_freqs"] = bfreqs
+        dump_outputs(dump_dir, outputs)
     total_ms, enc_ms, dec_ms = rig.max_over_ranks([t_start.elapsed_time(t_end),
                                                    float(np.mean([e[0].elapsed_time(e[1]) for e in ev])),
                                                    float(np.mean([e[1].elapsed_time(e[2]) for e in ev]))])
@@ -539,7 +568,8 @@ def measure_e2e(rig, workload, data, n, chunk, cap, n_chunks, model, coder, sb, 
 
 def run_ours(args, rank, local_rank, world):
     rig = Rig(rank, local_rank, world)
-    head = measure(rig, args.workload, args.size, args.chunk, args.steps, args.warmup, args.e2e_steps, headline=True)
+    head = measure(rig, args.workload, args.size, args.chunk, args.steps, args.warmup, args.e2e_steps, headline=True,
+                   dump_dir=args.dump_outputs)
     configs = {}
     want = args.configs == "all" or (args.configs == "auto" and args.workload == HEADLINE and args.size == 1 << 30)
     if want:

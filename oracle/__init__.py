@@ -23,14 +23,28 @@ _u64p = C.POINTER(C.c_uint64)
 CODER_WORD, CODER_BYTE, CODER_ALIAS, CODER_RANS64 = 0, 1, 2, 3
 
 
+def _reference_dir():
+    """The reference checkout make builds _ref/ from: $REF, else the Makefile's `REF ?=` default."""
+    if os.environ.get("REF"):
+        return os.environ["REF"]
+    with open(os.path.join(_HERE, "Makefile")) as f:
+        for line in f:
+            if line.startswith("REF ?="):
+                return line.split("?=", 1)[1].strip()
+    raise RuntimeError("oracle/Makefile defines no REF default")
+
+
+REFERENCE = _reference_dir()
+
+
 def build(force=False):
-    """Compile liboracle.so (always) and _ref/ (only if /root/reference is present)."""
+    """Compile liboracle.so (always) and _ref/ (only if the reference checkout REFERENCE is present)."""
     need = force or not os.path.exists(os.path.join(_HERE, "liboracle.so"))
     src = os.path.join(_HERE, "rans_oracle.c")
     lib = os.path.join(_HERE, "liboracle.so")
     if not need and os.path.getmtime(src) > os.path.getmtime(lib):
         need = True
-    if need or (os.path.isdir("/root/reference") and not os.path.exists(os.path.join(_HERE, "_ref", "libryg_ref.so"))):
+    if need or (os.path.isdir(REFERENCE) and not os.path.exists(os.path.join(_HERE, "_ref", "libryg_ref.so"))):
         subprocess.check_call(["make", "-C", _HERE, "all"], stdout=subprocess.DEVNULL)
 
 

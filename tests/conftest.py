@@ -48,14 +48,6 @@ def oracle_lib():
 
 
 @pytest.fixture(scope="session")
-def ref_lib():
-    import oracle
-    if not oracle.Reference.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    return oracle.Reference()
-
-
-@pytest.fixture(scope="session")
 def cuda_box():
     """For GPU tests that drive the library from a child process: skip (rather than fail) where there is no GPU."""
     import torch

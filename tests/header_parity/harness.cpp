@@ -1,64 +1,54 @@
 // Function-level differential test of include/rans_byte.h, rans64.h, rans_word_sse41.h against the reference's headers.
-// REFDIR is replaced by the reference checkout's path at test time (tests/test_header_parity.py); nothing of the
-// reference is copied here -- its headers are #included where they lie, inside namespace ref.
+// body.inc drives every function of the three APIs and records everything observable; this harness prints one digest
+// line per API and seed.  tests/test_header_parity.py builds it against include/*.h and requires the lines the same
+// harness printed when built against the reference's own headers (-DRANS_REF_HEADERS, REFDIR replaced by the
+// reference checkout's path), which tests/golden/make_reference_vectors.py stored in tests/golden/reference_vectors.json.
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
 #include <stdio.h>
 #include <assert.h>
 #include <smmintrin.h>
-#include "REFDIR/platform.h"
 #include <algorithm>
 #include <random>
 #include <vector>
 
-namespace ref {
+#ifdef RANS_REF_HEADERS
+#include "REFDIR/platform.h"
 #include "REFDIR/rans_byte.h"
 #include "REFDIR/rans64.h"
 #include "REFDIR/rans_word_sse41.h"
-#include "body.inc"
-}
-#undef RANS_BYTE_HEADER
-#undef RANS64_HEADER
-#undef RANS_WORD_SSE41_HEADER
-#undef RansAssert
-#undef Rans64Assert
-#undef RANS_BYTE_L
-#undef RANS64_L
-#undef RANS_WORD_L
-#undef RANS_WORD_SCALE_BITS
-#undef RANS_WORD_M
-#undef RANS_WORD_NSYMS
-namespace ours {
+#else
+#include "platform.h"
 #include "rans_byte.h"
 #include "rans64.h"
 #include "rans_word_sse41.h"
+#endif
 #include "body.inc"
+
+// FNV-1a, 64 bit: one digest over the recorded values, one over the produced stream bytes
+static uint64_t fnv1a(const void* p, size_t n)
+{
+    const uint8_t* q = (const uint8_t*)p;
+    uint64_t h = 0xcbf29ce484222325ull;
+    for (size_t i = 0; i < n; i++) h = (h ^ q[i]) * 0x100000001b3ull;
+    return h;
 }
 
-template <class A, class B> static int cmp(const char* what, const A& a, const B& b)
+static void report(const char* what, uint64_t seed, const Out& o)
 {
-    if (!a.round_trips || !b.round_trips) { printf("%s: a decode did not reproduce its input (ref %d, ours %d)\n", what, (int)a.round_trips, (int)b.round_trips); return 1; }
-    if (a.bytes != b.bytes || a.vals != b.vals) {
-        size_t i = 0;
-        while (i < a.vals.size() && i < b.vals.size() && a.vals[i] == b.vals[i]) i++;
-        printf("%s DIFFERS: %zu/%zu values, %zu/%zu bytes, first value mismatch at %zu\n", what, a.vals.size(), b.vals.size(),
-               a.bytes.size(), b.bytes.size(), i);
-        for (size_t k = (i > 8 ? i - 8 : 0); k < i + 6 && k < a.vals.size(); k++) printf("  [%zu] ref=%llx ours=%llx\n", k, (unsigned long long)a.vals[k], (unsigned long long)b.vals[k]);
-        printf("  bytes equal: %d\n", (int)(a.bytes == b.bytes));
-        return 1;
-    }
-    printf("%s ok: %zu values, %zu stream bytes identical\n", what, a.vals.size(), a.bytes.size());
-    return 0;
+    printf("%s seed %llu: round trips %d, %zu values fnv1a %016llx, %zu stream bytes fnv1a %016llx\n", what,
+           (unsigned long long)seed, (int)o.round_trips, o.vals.size(),
+           (unsigned long long)fnv1a(o.vals.data(), o.vals.size() * sizeof(uint64_t)), o.bytes.size(),
+           (unsigned long long)fnv1a(o.bytes.data(), o.bytes.size()));
 }
 
 int main()
 {
-    int bad = 0;
     for (uint64_t seed = 1; seed <= 3; seed++) {
-        { ref::Out a; ours::Out b; ref::run_byte(seed, a); ours::run_byte(seed, b); bad += cmp("rans_byte.h", a, b); }
-        { ref::Out a; ours::Out b; ref::run_64(seed, a); ours::run_64(seed, b); bad += cmp("rans64.h", a, b); }
-        { ref::Out a; ours::Out b; ref::run_word(seed, a); ours::run_word(seed, b); bad += cmp("rans_word_sse41.h", a, b); }
+        { Out o; run_byte(seed, o); report("rans_byte.h", seed, o); }
+        { Out o; run_64(seed, o); report("rans64.h", seed, o); }
+        { Out o; run_word(seed, o); report("rans_word_sse41.h", seed, o); }
     }
-    return bad;
+    return 0;
 }

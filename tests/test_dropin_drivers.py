@@ -4,7 +4,7 @@ platform.h) and print the reference's known-answer sizes and 'decode ok!'.
 
 The drivers are copied to a temp dir at test time (a quoted #include looks beside the
 including file first, so they cannot be compiled in place) -- nothing from the reference is
-ever copied into the repo.  Needs /root/reference, so it runs in the build container only.
+ever copied into the repo.  So that test needs the reference checkout (oracle.REFERENCE).
 """
 import os
 import re
@@ -13,10 +13,10 @@ import subprocess
 
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+import oracle
 
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "book1")), reason="reference checkout not present")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = oracle.REFERENCE
 
 DRIVERS = [
     ("main.cpp", [], [435113, 435117]),                    # README:48,62
@@ -26,6 +26,7 @@ DRIVERS = [
 ]
 
 
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "book1")), reason="needs the reference's driver sources")
 @pytest.mark.parametrize("src,flags,sizes", DRIVERS)
 def test_reference_driver_builds_unchanged_and_round_trips(tmp_path, src, flags, sizes):
     shutil.copy(os.path.join(REF, src), tmp_path / src)

@@ -4,6 +4,10 @@ Mirrors the reference's own verification (decode-output memcmp, main_simd.cpp:34
 and strengthens it: the GPU blob must equal the oracle's container byte for byte, the
 GPU must decode the oracle's blob, and the oracle must decode the GPU's blob.
 """
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -11,11 +15,36 @@ import oracle as orc
 
 pytestmark = pytest.mark.gpu
 
+# the reference's own N = 32 streams of the inputs below (tests/golden/make_reference_vectors.py)
+REF_N32 = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_vectors.json")))["n32"]
+
 WORD, BYTE, ALIAS, RANS64 = 0, 1, 2, 3
 
 
 def _model(oracle_lib, data, scale_bits):
     return oracle_lib.model(data, scale_bits)
+
+
+def _sha(*arrays):
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def _reference_stream_n32(gpu_ctx, oracle_lib, data, coder, ocoder, sb, want):
+    """One chunk of the GPU container is the reference's N = 32 stream: same model, same bytes (size and SHA-256 of
+    the reference's stream), and it decodes in exactly the bytes the reference's decoder consumed."""
+    assert _sha(data) == want["data_sha256"]
+    freqs, cum = oracle_lib.model(data, sb)
+    assert _sha(freqs, cum) == want["model_sha256"]
+    model = gpu_ctx.model(coder, sb, freqs)
+    blob, offs = gpu_ctx.encode_host(model, data, 1 << 16)
+    stream = blob[int(offs[0]):]
+    assert stream.size == want["bytes"] and _sha(stream) == want["sha256"]
+    dec, used = oracle_lib.decode(ocoder, stream, data.size, freqs, cum, 32, sb)
+    assert np.array_equal(dec, data) and used == want["used"] == stream.size
+    model.close()
 
 
 def _roundtrip(gpu_ctx, oracle_lib, data, coder, scale_bits, chunk):
@@ -51,17 +80,9 @@ def test_word_empty(gpu_ctx, oracle_lib, gen):
     assert out.size == 0
 
 
-def test_word_reference_stream_n32(gpu_ctx, oracle_lib, ref_lib, gen):
+def test_word_reference_stream_n32(gpu_ctx, oracle_lib, gen):
     """A single chunk IS the reference's N-way stream with N = 32 (SURVEY 8a layout)."""
-    data = gen("text", 50000, 5)
-    freqs, cum = ref_lib.model(data, 12)
-    ref_stream = ref_lib.encode(orc.CODER_WORD, data, freqs, cum, 32)
-    model = gpu_ctx.model(WORD, 12, freqs)
-    blob, offs = gpu_ctx.encode_host(model, data, 1 << 16)
-    assert np.array_equal(blob[int(offs[0]):], ref_stream)
-    # and the reference's own primitives decode the GPU stream
-    dec, used = ref_lib.decode(orc.CODER_WORD, blob[int(offs[0]):], data.size, freqs, cum, 32)
-    assert np.array_equal(dec, data) and used == ref_stream.size
+    _reference_stream_n32(gpu_ctx, oracle_lib, gen("text", 50000, 5), WORD, orc.CODER_WORD, 12, REF_N32["word"])
 
 
 def test_book1_known_answer_through_the_gpu(gpu_ctx, oracle_lib):
@@ -146,15 +167,8 @@ def test_alias_parity(gpu_ctx, oracle_lib, gen, kind, n, chunk, sb):
     _roundtrip(gpu_ctx, oracle_lib, data, ALIAS, sb, chunk)
 
 
-def test_alias_reference_stream_n32(gpu_ctx, ref_lib, gen):
-    data = gen("zipf", 60000, 6)
-    freqs, cum = ref_lib.model(data, 16)
-    ref_stream = ref_lib.encode(orc.CODER_ALIAS, data, freqs, cum, 32, 16)
-    model = gpu_ctx.model(ALIAS, 16, freqs)
-    blob, offs = gpu_ctx.encode_host(model, data, 1 << 16)
-    assert np.array_equal(blob[int(offs[0]):], ref_stream)
-    dec, used = ref_lib.decode(orc.CODER_ALIAS, blob[int(offs[0]):], data.size, freqs, cum, 32, 16)
-    assert np.array_equal(dec, data) and used == ref_stream.size
+def test_alias_reference_stream_n32(gpu_ctx, oracle_lib, gen):
+    _reference_stream_n32(gpu_ctx, oracle_lib, gen("zipf", 60000, 6), ALIAS, orc.CODER_ALIAS, 16, REF_N32["alias"])
 
 
 def test_alias_corrupt_stream_is_reported(gpu_ctx, oracle_lib, gen):
@@ -200,17 +214,11 @@ def test_rans64_parity(gpu_ctx, oracle_lib, gen, kind, n, chunk, sb):
 
 
 @pytest.mark.parametrize("coder,ocoder,sb", [(BYTE, orc.CODER_BYTE, 14), (RANS64, orc.CODER_RANS64, 14)])
-def test_byte_and_rans64_reference_stream_n32(gpu_ctx, ref_lib, gen, coder, ocoder, sb):
+def test_byte_and_rans64_reference_stream_n32(gpu_ctx, oracle_lib, gen, coder, ocoder, sb):
     """The reference's own RansEncPutSymbol / Rans64EncPutSymbol loops (N = 32) produce the GPU's chunk stream,
-    and the reference's decoders read the GPU stream."""
-    data = gen("text", 60000, 8)
-    freqs, cum = ref_lib.model(data, sb)
-    ref_stream = ref_lib.encode(ocoder, data, freqs, cum, 32, sb)
-    model = gpu_ctx.model(coder, sb, freqs)
-    blob, offs = gpu_ctx.encode_host(model, data, 1 << 16)
-    assert np.array_equal(blob[int(offs[0]):], ref_stream)
-    dec, used = ref_lib.decode(ocoder, blob[int(offs[0]):], data.size, freqs, cum, 32, sb)
-    assert np.array_equal(dec, data) and used == ref_stream.size
+    and it decodes in exactly the bytes the reference's decoders consumed."""
+    _reference_stream_n32(gpu_ctx, oracle_lib, gen("text", 60000, 8), coder, ocoder, sb,
+                          REF_N32["byte" if coder == BYTE else "rans64"])
 
 
 # ---------------------------------------------------------------- device histogram / per-block models (config 5)
